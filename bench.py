@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's B200 path (one rank per GPU under torchrun)
     python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU path (oracle port) on the host cores
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR   # B200 path: also save what the last timed step computed
 
 Prints ONE JSON line (rank 0).  Workload = BASELINE.json configs[2] ("image_inpainting.py PartialConv UNet
 @512x512 batch=8, 1xB200 fwd+bwd bf16"), the configuration the headline metric is quoted on; weak scaling
@@ -48,7 +49,15 @@ def parse():
     ap.add_argument("--no-graph", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--profile-layers", action="store_true", help="print a per-layer CUDA-event table to stderr")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="B200 path only: after the timed steps, write what the last one computed to DIR/<name>.npy "
+                         "(see dump_outputs)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs saves the outputs of the b200 path")
+    return args
 
 
 # --------------------------------------------------------------------------------------------------
@@ -139,40 +148,10 @@ def pick_threads():
     return best, cores
 
 
-_REF_CACHE = {}
-
-
-def _reference_module():
-    """The UNMODIFIED reference's models.image_inpainting (from /root/reference in the build container, from the staging copy
-    baseline/_ref on the GPU box -- tools/stage_reference.py), or None when neither exists."""
-    if "mod" in _REF_CACHE:
-        return _REF_CACHE["mod"]
-    _REF_CACHE["mod"] = None
-    sys.path.insert(0, os.path.join(ROOT, "tools"))
-    try:
-        from stage_reference import reference_dir
-        ref = reference_dir()
-    except Exception:  # noqa: BLE001
-        ref = None
-    if ref is None or "models" in sys.modules:
-        return None
-    sys.path.insert(0, ref)
-    try:
-        import importlib
-        _REF_CACHE["mod"] = importlib.import_module("models.image_inpainting")
-        return _REF_CACHE["mod"]
-    except Exception as exc:  # noqa: BLE001
-        print(f"[bench] importing the staged reference failed ({type(exc).__name__}: {exc}); using the oracle port", file=sys.stderr)
-        return None
-    finally:
-        sys.path.remove(ref)
-
-
 def cpu_reference_steps(steps, warmup, batch=1, seed=0, workload="unet"):
-    """fwd + bwd + SGD of ImageFillOrigin on the host cores.  kind "reference": the reference's own nn.Modules
-    (models/image_inpainting.py + models/partial_convolution.py, stock torch CPU code path, nothing of this repo on the path);
-    kind "port": the oracle's functional restatement (same ATen ops in the same order; pinned bit-exactly by tests/golden) when the
-    reference is not staged.  Returns (images_per_sec, ms_per_step, cores, kind)."""
+    """fwd + bwd + SGD of the workload's network on the host cores, computed by the oracle's functional restatement of the
+    reference (same ATen ops in the same order; pinned bit-exactly by tests/golden).  Returns (images_per_sec, ms_per_step,
+    cores, kind)."""
     import torch
 
     from text_segmentation_image_inpainting_b200.synthetic import random_hole_masks
@@ -182,33 +161,19 @@ def cpu_reference_steps(steps, warmup, batch=1, seed=0, workload="unet"):
     x = torch.randn(batch, 3, HW, HW)
     mask = torch.from_numpy(random_hole_masks(batch, HW, HW, seed=seed))
     xin = x * mask
-    ref = _reference_module()
+    kind = "port"
     if workload != "unet":
         import contextlib
         import io
         cls = {"textseg": "TextSegament", "xception": "XceptionTextSegment"}[workload]
         with contextlib.redirect_stdout(io.StringIO()):
-            if ref is not None:
-                kind = "reference"
-                import importlib
-                net = getattr(importlib.import_module("models.text_segmentation"), cls)().train()
-                params = [p for p in net.parameters() if p.requires_grad]
-                fwd = lambda: net(x)                                       # noqa: E731
-            else:
-                kind = "port"
-                from oracle import seg_torch as OS                     # cpu_baseline leg: allowed importer of oracle/
-                from oracle.pconv_torch import clone_state_dict
-                from text_segmentation_image_inpainting_b200.models import text_segmentation as MT
-                sd = clone_state_dict(getattr(MT, cls)().state_dict(), requires_grad=True)
-                params = [v for v in sd.values() if v.requires_grad]
-                fwd = lambda: OS.NETWORKS[cls](sd, x)                      # noqa: E731
-    elif ref is not None:
-        kind = "reference"
-        net = ref.ImageFillOrigin().train()
-        params = [p for p in net.parameters() if p.requires_grad]
-        fwd = lambda: net((xin, mask))                                 # noqa: E731
+            from oracle import seg_torch as OS                         # cpu_baseline leg: allowed importer of oracle/
+            from oracle.pconv_torch import clone_state_dict
+            from text_segmentation_image_inpainting_b200.models import text_segmentation as MT
+            sd = clone_state_dict(getattr(MT, cls)().state_dict(), requires_grad=True)
+            params = [v for v in sd.values() if v.requires_grad]
+            fwd = lambda: OS.NETWORKS[cls](sd, x)                          # noqa: E731
     else:
-        kind = "port"
         from oracle import pconv_torch as O                       # cpu_baseline leg: allowed importer of oracle/
         from text_segmentation_image_inpainting_b200.models.image_inpainting import ImageFillOrigin
         skeleton = ImageFillOrigin()                               # parameter names / shapes / default init only
@@ -240,7 +205,7 @@ def run_reference(args):
         "impl": "reference", "metric": W["metric"], "value": ips, "unit": "images/sec", "n_gpus": args.gpus, "steps": args.steps,
         "warmup": args.warmup, "ms_per_step": ms, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
         "dtype": "f32", "data": "synthetic",
-        "config": {"workload": W["label"] + " 512x512 fwd+bwd+SGD, CPU (" + ("the unmodified reference's own modules" if kind == "reference" else "reference algorithm via the oracle port") + ")",
+        "config": {"workload": W["label"] + " 512x512 fwd+bwd+SGD, CPU (reference algorithm via the oracle port)",
                    "batch_per_step": 1, "note": f"each step is a bounded sample (1 image) of the batch-{W['batch']} workload"},
         "cpu_baseline": {"value": ips, "unit": "images/sec", "cores": cores_n, "cores_note": cores, "kind": kind,
                          "sample": f"{args.steps} steps x 1 image @512x512 after {args.warmup} warm-up"},
@@ -340,6 +305,32 @@ def layer_profile(ts, x, mask, peaks, verbose):
         except Exception:  # noqa: BLE001
             pass
     return roof, fam, roofs
+
+
+DUMP_MAX_ELEMS = 1 << 22          # per array (16 MB of float32): the four arrays of a dump stay under 64 MB together
+
+
+def dump_outputs(out_dir, loss, net):
+    """Save what the last timed step handed back, so that two builds can be compared output for output on identical inputs:
+    loss.npy (float64, the step's loss), and the model the step left behind as float32 vectors -- params.npy (parameters after
+    the SGD update), grads.npy (the step's gradients) and bn_stats.npy (floating-point buffers: BatchNorm running statistics).
+    Each vector concatenates its tensors in named_parameters() / named_buffers() order, every tensor flattened in logical NCHW
+    order.  A vector longer than DUMP_MAX_ELEMS is replaced by a fixed sample: the elements at DUMP_MAX_ELEMS sorted indices
+    drawn without replacement by numpy's default_rng(0), which depend only on the vector's length."""
+    import numpy as np
+    import torch
+
+    def flat(tensors):
+        return torch.cat([t.detach().float().reshape(-1).cpu() for t in tensors]).numpy()
+
+    params = [p for p in net.parameters() if p.requires_grad]
+    arrays = {"loss": np.array([float(loss)], dtype=np.float64), "params": flat(params), "grads": flat(p.grad for p in params),
+              "bn_stats": flat(b for b in net.buffers() if b.is_floating_point())}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        if a.size > DUMP_MAX_ELEMS:
+            a = a[np.sort(np.random.default_rng(0).choice(a.size, DUMP_MAX_ELEMS, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def run_b200(args):
@@ -462,16 +453,20 @@ def run_b200(args):
             consumed[b].record()
             loss_host.copy_(loss, non_blocking=True)
         torch.cuda.current_stream().synchronize()
+        return loss
 
     e2e_run(max(2, min(args.warmup, 3)))
     barrier()
     e0.record()
-    e2e_run(args.steps)
+    last_loss = e2e_run(args.steps)
     e1.record()
     barrier()
     e2e_ms = maxreduce(e0.elapsed_time(e1))
     e2e_value = world * B * args.steps / (e2e_ms * 1e-3)
     note("end-to-end done")
+    if args.dump_outputs and rank == 0:
+        # before the instrumented eager step below, which recomputes the gradients
+        dump_outputs(args.dump_outputs, last_loss, net)
 
     # ---------------- per-kernel roofline (rank 0): eager instrumented step, events on the launching stream
     roof, fam, roofs = (None, {}, {})

@@ -8,16 +8,14 @@ if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
 GOLDEN = os.path.join(ROOT, "tests", "golden")
-REFERENCE = os.environ.get("PCB_REFERENCE", "/root/reference")
+GOLDEN_THREADS = 8
 
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box with -m gpu)")
-    config.addinivalue_line("markers", "reference: needs /root/reference (build container only)")
 
 
 def pytest_collection_modifyitems(config, items):
-    have_ref = os.path.isdir(os.path.join(REFERENCE, "models"))
     try:
         import torch
         have_gpu = torch.cuda.is_available()
@@ -29,8 +27,6 @@ def pytest_collection_modifyitems(config, items):
     for it in items:
         if have_timeout and "gpu" in it.keywords and it.get_closest_marker("timeout") is None:
             it.add_marker(pytest.mark.timeout(300, method="thread"))
-        if "reference" in it.keywords and not have_ref:
-            it.add_marker(pytest.mark.skip(reason="/root/reference not present on this box"))
         if "gpu" in it.keywords and not have_gpu:
             it.add_marker(pytest.mark.skip(reason="no CUDA device"))
 
@@ -38,3 +34,15 @@ def pytest_collection_modifyitems(config, items):
 @pytest.fixture(scope="session")
 def golden_dir():
     return GOLDEN
+
+
+@pytest.fixture(scope="module")
+def golden_threads():
+    """Bit-exact comparisons with the goldens run with the intra-op thread count the goldens were written with
+    (tests/golden/make_golden*.py): ATen's CPU convolutions and reductions split their sums by thread count, so on a host
+    that defaults to another count the last bits differ."""
+    import torch
+    saved = torch.get_num_threads()
+    torch.set_num_threads(GOLDEN_THREADS)
+    yield
+    torch.set_num_threads(saved)

@@ -119,6 +119,44 @@ def test_train_step_updates_match_oracle_sgd(dev):
     assert ref[-1] != ref[0]
 
 
+def test_bench_dump_outputs_writes_the_last_timed_step(tmp_path):
+    """`bench.py --dump-outputs DIR`: one JSON line, and float32 / float64 arrays of the last timed step (loss, updated parameters,
+    gradients, BatchNorm statistics) of at most 64 MB in all.  Two runs with the same arguments see the same inputs and so dump
+    the same values (up to the unordered fp32 adds of the weight gradients); one more timed step moves the dumped state."""
+    import json
+
+    import numpy as np
+    from text_segmentation_image_inpainting_b200.models.image_inpainting import ImageFillOrigin
+
+    def run(steps, name):
+        out = tmp_path / name
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--gpus", "1", "--steps", str(steps), "--warmup", "1",
+                            "--no-cpu-baseline", "--dump-outputs", str(out)], capture_output=True, text=True, timeout=90, cwd=ROOT)
+        assert r.returncode == 0, r.stderr[-3000:]
+        lines = [ln for ln in r.stdout.splitlines() if ln.strip()]
+        assert len(lines) == 1 and json.loads(lines[0])["steps"] == steps, r.stdout[:500]
+        assert sum(f.stat().st_size for f in out.iterdir()) <= 64 << 20
+        return {f.stem: np.load(f) for f in out.iterdir()}
+
+    one, two, again = run(1, "one"), run(2, "two"), run(2, "again")
+    assert set(two) == {"loss", "params", "grads", "bn_stats"}
+    assert all(a.dtype in (np.float32, np.float64) and np.isfinite(a).all() for a in two.values())
+    n_params = sum(p.numel() for p in ImageFillOrigin().parameters() if p.requires_grad)
+    assert two["params"].shape == two["grads"].shape == (min(n_params, 1 << 22),)
+    assert two["loss"].shape == (1,) and two["loss"][0] > 0 and np.abs(two["grads"]).max() > 0
+
+    def diff(a, b, name):
+        return float(np.abs(a[name].astype(np.float64) - b[name]).max())
+    # same arguments: same inputs, same trajectory
+    assert diff(two, again, "loss") <= 1e-3 * abs(float(two["loss"][0])), (two["loss"], again["loss"])
+    for name in ("params", "grads", "bn_stats"):
+        assert diff(two, again, name) <= 1e-3 * float(np.abs(two[name]).max()), name
+    # --steps sets the number of timed (optimiser) steps: one more step moves the parameters and the loss by far more than
+    # the run-to-run noise above
+    assert diff(one, two, "params") > 100 * diff(two, again, "params")
+    assert diff(one, two, "loss") > 100 * diff(two, again, "loss")
+
+
 # ------------------------------------------------------------------------------------------------------------------
 # two ranks over NCCL: the averaged gradient arena == the single-process gradient of the concatenated batch
 # ------------------------------------------------------------------------------------------------------------------

@@ -63,10 +63,14 @@ SEG_GOLDENS = [("TextSegament", ""), ("XceptionTextSegment", ""), ("TextSegament
 def test_network_fp32_matches_reference_golden(cls_name, tag, dev):
     """exact mode end to end: forward within 1e-3 relative of the reference's CPU forward (north_star bar);
     gradients within 2e-3 (fp32 re-association noise amplified by the tiny-batch BatchNorms at the bottom)."""
+    from text_segmentation_image_inpainting_b200 import ops
+    before = ops.LAZYCAT_MATERIALIZED
     errs = run_net(cls_name, dev, F32, tag)
     worst = sorted(errs.items(), key=lambda kv: -kv[1])[:4]
     assert errs["out"] <= 1e-3 and errs["out_row"] <= 1e-3 and errs["loss"] <= 1e-5, worst
     assert max(errs.values()) <= (5e-3 if tag == "_512" else 2e-3), worst
+    # the decoder's upsample + skip concatenation stayed lazy: no upsample / concat pass ran
+    assert ops.LAZYCAT_MATERIALIZED == before
 
 
 @pytest.mark.parametrize("cls_name,tag", NET_GOLDENS)
@@ -74,9 +78,12 @@ def test_network_bf16_tensor_core_mode(cls_name, tag, dev):
     """bf16 storage + tcgen05: 16+ layers of bf16 rounding -> a few 1e-3 on the output and loss.  Gradients of the
     BatchNorm scales see LeakyReLU sign flips of pre-activations within one bf16 ulp of zero (a systematic, not a
     random, perturbation): a few percent of max|grad|; convolution weight grads stay at the 1e-3 level."""
+    from text_segmentation_image_inpainting_b200 import ops
+    before = ops.LAZYCAT_MATERIALIZED
     errs = run_net(cls_name, dev, BF, tag)
     worst = sorted(errs.items(), key=lambda kv: -kv[1])[:6]
     assert _pipeline_clean()
+    assert ops.LAZYCAT_MATERIALIZED == before         # the decoder's upsample + skip concatenation stayed lazy
     # forward / loss / running statistics against the fp32 REFERENCE golden
     assert errs["out"] <= 2e-2 and errs["loss"] <= 2e-3, worst
     assert all(v <= 2e-2 for k, v in errs.items() if k.startswith("bn.")), worst

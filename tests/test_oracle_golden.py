@@ -13,6 +13,8 @@ from oracle.pconv_box import pconv_box_forward
 
 from conftest import GOLDEN
 
+pytestmark = pytest.mark.usefixtures("golden_threads")
+
 L1 = sorted(os.path.basename(p)[:-4] for p in glob.glob(os.path.join(GOLDEN, "pc_*.npz")))
 
 

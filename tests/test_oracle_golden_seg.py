@@ -19,6 +19,8 @@ from text_segmentation_image_inpainting_b200.models import MobileNetV2 as MM
 from text_segmentation_image_inpainting_b200.models import common as MC
 from text_segmentation_image_inpainting_b200.models import text_segmentation as MT
 
+pytestmark = pytest.mark.usefixtures("golden_threads")
+
 ACT = ("leaky", 0.3)
 
 
